@@ -214,6 +214,30 @@ def pin_batch(batch):
     return {k: (v.pin_memory() if torch.is_tensor(v) else v) for k, v in batch.items()}
 
 
+DUMP_PER_PARAM = 4096       # sampled elements per parameter tensor: 1.2M in all on the R2R model (4.7 MB)
+
+
+def dump_outputs(out_dir, loss, model, opt):
+    """Writes what the last timed step computed as float32 .npy files under `out_dir`: its loss, the total gradient
+    norm it clipped with (own AdamW only) and the parameters it left behind, sampled at fixed, seeded DUMP_PER_PARAM
+    positions of every parameter (all of a smaller one) and concatenated in `named_parameters()` order.  fp32 atomics in
+    the weight-gradient reductions make the step differ from run to run in the last bits, and the steps before it
+    amplify that (B200 at 1000 W, R2R, --steps 22 --warmup 5: loss up to 1e-2, gradient norm 5e-2 and parameters
+    3e-4 relative apart)."""
+    import numpy as np
+    params = [p for _, p in model.named_parameters()]
+    idx = [torch.arange(p.numel()) if p.numel() <= DUMP_PER_PARAM else
+           torch.randint(p.numel(), (DUMP_PER_PARAM,), generator=torch.Generator().manual_seed(i))
+           for i, p in enumerate(params)]
+    out = {"loss": loss.detach().reshape(-1),
+           "params": torch.cat([p.detach().reshape(-1)[j.to(p.device)] for p, j in zip(params, idx)])}
+    if not isinstance(opt, torch.optim.Optimizer):
+        out["grad_norm"] = opt.total_grad_norm().reshape(-1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args, rank, world, local_rank):
     import torch.distributed as dist
     from bevbert_b200 import kernels as K
@@ -337,7 +361,7 @@ def run_ours(args, rank, world, local_rank):
     host_t0 = time.perf_counter()
     e0.record()
     for i in range(args.steps):
-        train_step(resident[MIX[i % len(MIX)]][i % 2], MIX[i % len(MIX)])
+        loss = train_step(resident[MIX[i % len(MIX)]][i % 2], MIX[i % len(MIX)])
     e1.record()
     host_enqueue_ms = (time.perf_counter() - host_t0) * 1e3 / args.steps     # host time to enqueue a step
     sync_all()
@@ -353,6 +377,8 @@ def run_ours(args, rank, world, local_rank):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t)
     value = Bs * world * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, model, opt)
 
     # ------------------------------------------------------------------ end to end: pinned host -> device each step
     # Static device input buffers (one set per resident batch), filled from pinned host memory on a copy stream one
@@ -543,8 +569,18 @@ def main():
     ap.add_argument("--ddp", action="store_true", help="wrap with torch DDP instead of the flat gradient all-reduce")
     ap.add_argument("--strong", action="store_true",
                     help="strong scaling: --batch is the GLOBAL batch, split over the ranks (default: weak, --batch per GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last one's loss, gradient norm and a fixed sample of the "
+                         "parameters it left behind to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3)
+    # dropout masks derive from torch's seed (blocks.Runtime, graphs.GraphedTrainStep): fixed, so that runs with the
+    # same arguments compute the same step
+    torch.manual_seed(0)
     global WORKLOAD, MIX
     WORKLOAD = args.config
     MIX = list(WORKLOADS[WORKLOAD]["mix"])

@@ -6,10 +6,10 @@ A plain-PyTorch *functional* restatement of the reference's algorithm, evaluated
 in bench.py (`cpu_baseline`, `--impl reference`), because the reference itself (/root/reference) cannot
 travel to the GPU box.  The product package never imports it.
 
-Pinned against the real reference: tests/test_oracle_vs_reference.py runs the unmodified reference
-modules (oracle/ref_shim.py) on the same weights/batches in the build container, and
-tests/golden/*.pt hold reference outputs for the GPU box.  The reference ships no tests or golden
-vectors of its own (SURVEY.md 4, 8c).
+Pinned against the real reference: tests/golden/make_golden.py runs the unmodified reference modules
+(oracle/ref_shim.py) on seeded weights/batches and stores their outputs in tests/golden/*.pt, which
+tests/test_oracle_golden.py and tests/test_oracle_vs_reference.py compare with.  The reference ships
+no tests or golden vectors of its own (SURVEY.md 4, 8c).
 
 Every function cites the reference lines it restates (paths relative to the reference root,
 pretrain_src/model/...).  Dropout is taken as p = 0 unless `drop_p` is given (parity runs use 0).

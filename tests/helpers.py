@@ -1,8 +1,41 @@
 """Shared helpers for the parity tests."""
+import contextlib
+import hashlib
+
 import torch
 
 from bevbert_b200 import synth
 from bevbert_b200.config import make_config
+
+# tests/golden/make_golden.py runs the reference with this many intra-op threads.  torch splits fp32 reductions on the
+# CPU by thread count, so the oracle reproduces the stored outputs bit for bit only with the same count.
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    prev = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(prev)
+
+
+def golden_sample(t, n=8192):
+    """n elements of `t` at fixed positions (synth's reproducible generator): what tests/golden/ keeps of an output too
+    large to store whole."""
+    flat = t.detach().reshape(-1)
+    return flat[synth.det_randint((n,), 0, 0, 0, flat.numel() - 1)].clone()
+
+
+def digest(t):
+    """SHA-256 of a tensor's dtype, shape and bytes: a bit-exact comparison with an output too large to store."""
+    t = t.detach().contiguous()
+    h = hashlib.sha256(("%s %s " % (t.dtype, tuple(t.shape))).encode())
+    h.update(t.view(torch.uint8).reshape(-1).numpy().tobytes())
+    return h.hexdigest()
+
 
 SMALL = dict(num_l_layers=2, num_x_layers=2, num_pano_layers=1, vocab_size=3000, bev_dim=11, bev_res=1.0,
              hidden_dropout_prob=0.0, attention_probs_dropout_prob=0.0, feat_dropout=0.0)

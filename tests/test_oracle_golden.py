@@ -7,9 +7,16 @@ import torch
 
 from bevbert_b200 import synth
 from bevbert_b200.model.pretrain_cmt import GlocalTextPathCMTPreTraining
+from helpers import golden_threads
 from oracle import bevbert_ref as R
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+@pytest.fixture(autouse=True)
+def _golden_threads():
+    with golden_threads():
+        yield
 
 
 def _cases():
